@@ -165,7 +165,7 @@ def _reference_engine_leg(msgs, seconds: float = 4.0):
     from detectmateservice_b200.synth import MONITORED_KEYS
     from oracle import ref_engine, rtok
     if ref_engine.reference_path() is None:
-        return {"unavailable": "reference service neither in baseline/_ref nor in /root/reference/src"}
+        return {"unavailable": "reference service not in oracle/_ref (make -C oracle ref)"}
     train = rtok.split_records(msgs[0][:LINE_BYTES * 2000])
     # (anomaly-free records: an alert would be answered on the feeder's socket)
     detect = rtok.split_records(msgs[0][LINE_BYTES * 2000:LINE_BYTES * 6000])
@@ -231,11 +231,11 @@ def _component(device: int, max_batch_bytes: int):
 
 def _config3_engine(h_msgs, nbytes, device: int, seconds: float = 2.0):
     """BASELINE config 3: sender -> NNG PAIR0 (ipc) -> DetectorEngine(B200NewValueDetector) -> sink."""
-    import tempfile
     import pynng
+    from detectmateservice_b200.compat import ipc_tempdir
     from detectmateservice_b200.service import DetectorEngine
     comp = _component(device, max(nbytes) + 4096)
-    tmp = tempfile.mkdtemp(prefix="dmcfg3")
+    tmp = ipc_tempdir("dmcfg3")
     eng_addr, out_addr = f"ipc://{tmp}/det.ipc", f"ipc://{tmp}/out.ipc"
     sink = pynng.Pair0(listen=out_addr, recv_timeout=30000)
     lines = [0]
@@ -282,6 +282,14 @@ def _config3_engine(h_msgs, nbytes, device: int, seconds: float = 2.0):
         sink.close()
         comp.close()
     return res
+
+
+def _dump_outputs(out_dir: str, rank: int, world: int, arrays: dict) -> None:
+    """--dump-outputs: DIR/<name>.npy for every array (DIR/<name>_rank<r>.npy when n_gpus > 1)."""
+    os.makedirs(out_dir, exist_ok=True)
+    sfx = f"_rank{rank}" if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{sfx}.npy"), a)
 
 
 def run_gpu(args):
@@ -337,6 +345,11 @@ def run_gpu(args):
     cap = LINES_PER_MSG + 16
     d_flags = torch.zeros(cap, dtype=torch.uint8, device=dev)
     d_scores = torch.zeros(cap, dtype=torch.float32, device=dev)
+    # the timed steps give every message of a window its own result rows: after a step the caller holds the flags and
+    # scores of all of its messages
+    w_flags = torch.zeros((WINDOW_MSGS, cap), dtype=torch.uint8, device=dev)
+    w_scores = torch.zeros((WINDOW_MSGS, cap), dtype=torch.float32, device=dev)
+    w_out = [(w_flags[m].data_ptr(), w_scores[m].data_ptr()) for m in range(WINDOW_MSGS)]
     from detectmateservice_b200.window import DeviceWindow
     dwin = DeviceWindow(det, rank, world, dev)
     if world > 1 and os.environ.get("DM_WINDOW", "native") == "native":
@@ -372,7 +385,7 @@ def run_gpu(args):
         n = 0
         for m in range(WINDOW_MSGS):
             j = 1 + ((i * WINDOW_MSGS + m) % N_DETECT)
-            det.enqueue_device(d_msgs[j].data_ptr(), nbytes[j], 0, d_flags.data_ptr(), d_scores.data_ptr(), cap, sp)
+            det.enqueue_device(d_msgs[j].data_ptr(), nbytes[j], 0, w_out[m][0], w_out[m][1], cap, sp)
             n += n_lines_msg[j]
         if world > 1:
             window(False)
@@ -402,6 +415,11 @@ def run_gpu(args):
     barrier()
     ms = e0.elapsed_time(e1)
     _, _, launches1 = det.profile_read()
+    if args.dump_outputs:                            # the last timed step's results, before the steps below overwrite them
+        last = [1 + (((args.steps - 1) * WINDOW_MSGS + m) % N_DETECT) for m in range(WINDOW_MSGS)]
+        _dump_outputs(args.dump_outputs, rank, world, {
+            "flags": np.stack([w_flags[m, :n_lines_msg[j]].cpu().numpy() for m, j in enumerate(last)]).astype(np.float32),
+            "scores": np.stack([w_scores[m, :n_lines_msg[j]].cpu().numpy() for m, j in enumerate(last)])})
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     tot = torch.tensor([float(lines_timed)], dtype=torch.float64, device=dev)
     if world > 1:
@@ -625,7 +643,14 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline legs")
     ap.add_argument("--no-extra", action="store_true", help="skip the config 3 / config 5 legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's results to DIR: flags.npy and scores.npy, float32, one row per "
+                         "message of the window (%d x %d records)" % (WINDOW_MSGS, LINES_PER_MSG))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if os.environ.get("DM_BENCH_WATCHDOG"):                    # a hung run says where: all threads' stacks every N seconds
         import faulthandler
         faulthandler.dump_traceback_later(float(os.environ["DM_BENCH_WATCHDOG"]), repeat=True, file=sys.stderr)

@@ -11,8 +11,15 @@ from __future__ import annotations
 import importlib
 import os
 import sys
+import tempfile
 
 SHIMS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "shims")
+
+
+def ipc_tempdir(prefix: str = "dm") -> str:
+    """A new directory for ``ipc://`` socket files.  An AF_UNIX address holds at most 107 bytes, which a deep
+    $TMPDIR can leave no room for, so the directory is made under /tmp where that exists."""
+    return tempfile.mkdtemp(prefix=prefix, dir="/tmp" if os.path.isdir("/tmp") else None)
 
 
 def install_shims() -> dict:

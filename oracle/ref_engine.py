@@ -2,8 +2,8 @@
 the CPU oracle as its library component (BASELINE.md section 4).  MEASUREMENT INFRASTRUCTURE:
 only bench.py's CPU legs and tests/ use this module.
 
-Where the reference comes from: `baseline/_ref` (pip --target install of the unmodified
-reference, travels to the GPU box) or /root/reference/src when that exists; its two missing
+Where the reference comes from: `oracle/_ref` (the unmodified reference service, put there by
+`make -C oracle ref` in build()); its two missing
 third-party imports (`pynng`, `detectmatelibrary.common.*`) are this repo's stand-ins
 (detectmateservice_b200/shims), real packages win when installed.
 
@@ -25,20 +25,17 @@ import time
 from typing import List, Optional, Tuple
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-_REF_CANDIDATES = [os.path.join(ROOT, "baseline", "_ref"), "/root/reference/src"]
+REF_DIR = os.path.join(ROOT, "oracle", "_ref")
 
 
 def reference_path() -> Optional[str]:
-    for p in _REF_CANDIDATES:
-        if os.path.isdir(os.path.join(p, "service")):
-            return p
-    return None
+    return REF_DIR if os.path.isdir(os.path.join(REF_DIR, "service")) else None
 
 
 def _setup_imports() -> str:
     p = reference_path()
     if p is None:
-        raise RuntimeError("the reference service is neither in baseline/_ref nor in /root/reference/src")
+        raise RuntimeError("the reference service is not in oracle/_ref (make -C oracle ref)")
     if ROOT not in sys.path:
         sys.path.insert(0, ROOT)
     if p not in sys.path:
@@ -174,8 +171,9 @@ def ipc_rate(keys: List[str], train_lines: List[bytes], detect_lines: List[bytes
              ) -> Tuple[float, int, float]:
     """records/s of n_services reference services (own process, own ipc socket, own feeder process):
     (aggregate rate, records timed, slowest feeder's seconds)."""
+    from detectmateservice_b200.compat import ipc_tempdir
     ctx = mp.get_context("spawn")
-    tmp = tempfile.mkdtemp(prefix="dmref")
+    tmp = ipc_tempdir("dmref")
     start = ctx.Event()
     done = ctx.Event()
     out_q = ctx.Queue()

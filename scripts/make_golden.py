@@ -16,10 +16,15 @@
   audit_templates.txt         the nine `<*>` templates of the reference's parser test data
                               (tests/library_integration/audit_templates.txt; test DATA, copied
                               verbatim as a fixture like audit_sample.log).
+  audit.log.gz                the full audit.log itself, gzip-compressed (test DATA).
+  schemas_descriptor.json     the FileDescriptorProto the reference embeds in
+                              container/fluentout/schemas_pb.rb:8, as hex.
 """
 import collections
+import gzip
 import json
 import os
+import re
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -35,11 +40,38 @@ KEYS = ["type", "exe", "terminal", "acct", "res"]
 N_TRAIN = 200
 
 
+def _ruby_unescape(s: str) -> bytes:
+    """The bytes of a double-quoted Ruby string literal's body."""
+    out = bytearray()
+    i = 0
+    simple = {"n": 10, "r": 13, "t": 9, '"': 34, "\\": 92, "e": 27, "a": 7, "b": 8, "f": 12, "v": 11, "0": 0, "#": 35}
+    while i < len(s):
+        c = s[i]
+        if c != "\\":
+            out += c.encode("latin-1")
+            i += 1
+            continue
+        n = s[i + 1]
+        if n == "x":
+            m = re.match(r"[0-9a-fA-F]{1,2}", s[i + 2:i + 4])
+            out.append(int(m.group(0), 16))
+            i += 2 + len(m.group(0))
+        elif n in "01234567":
+            m = re.match(r"[0-7]{1,3}", s[i + 1:i + 4])
+            out.append(int(m.group(0), 8))
+            i += 1 + len(m.group(0))
+        else:
+            out.append(simple[n])
+            i += 2
+    return bytes(out)
+
+
 def main() -> None:
     os.makedirs(OUT, exist_ok=True)
     with open(os.path.join(REF, "tests/library_integration/audit_templates.txt"), "rb") as f:
         open(os.path.join(OUT, "audit_templates.txt"), "wb").write(f.read())
     raw = open(os.path.join(REF, "tests/library_integration/audit.log"), "rb").read()
+    open(os.path.join(OUT, "audit.log.gz"), "wb").write(gzip.compress(raw, compresslevel=9, mtime=0))
     lines = rtok.split_records(raw)
     counts = collections.Counter(l.split(b" ")[0][5:].decode() for l in lines)
     rare = {t for t, c in counts.items() if c <= 4}
@@ -89,6 +121,11 @@ def main() -> None:
                      "description": "NewValueDetector detects values not encountered in training as anomalies.",
                      "alertsObtain": {"Global - URL": "Unknown value: '/foobar'"}}},
         open(os.path.join(OUT, "docs_golden.json"), "w"), indent=1)
+
+    rb = open(os.path.join(REF, "container/fluentout/schemas_pb.rb"), "r", encoding="latin-1").read()
+    lit = re.search(r'descriptor_data = "((?:[^"\\]|\\.)*)"', rb, re.S).group(1)
+    json.dump({"source": "container/fluentout/schemas_pb.rb:8 (descriptor_data)", "file_descriptor_hex": _ruby_unescape(lit).hex()},
+              open(os.path.join(OUT, "schemas_descriptor.json"), "w"), indent=1)
     print("golden written:", sorted(os.listdir(OUT)), "sample records:", len(pick), "anomalies:", sum(flags))
 
 

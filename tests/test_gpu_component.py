@@ -91,7 +91,7 @@ def test_raw_mode_alerts_audit_sample(golden_dir):
     comp.close()
 
 
-def test_engine_pipeline_raw_messages(tmp_path):
+def test_engine_pipeline_raw_messages(sock_dir):
     """sender -> [ipc] -> DetectorEngine(B200NewValueDetector) -> [ipc] -> sink, 64k-record messages
     (BASELINE config 3 topology at small scale)."""
     import pynng
@@ -108,7 +108,7 @@ def test_engine_pipeline_raw_messages(tmp_path):
         "params": {"output_format": "compact", "max_batch_bytes": 4 << 20},
         "global": {"g": {"header_variables": [{"pos": k} for k in MONITORED_KEYS]}}}}}
     comp = _comp(cfg)
-    eng_addr, out_addr = f"ipc://{tmp_path}/det.ipc", f"ipc://{tmp_path}/out.ipc"
+    eng_addr, out_addr = f"ipc://{sock_dir}/det.ipc", f"ipc://{sock_dir}/out.ipc"
     sink = pynng.Pair0(listen=out_addr, recv_timeout=20000)
     with DetectorEngine(comp, eng_addr, out_addr=[out_addr]) as eng:
         time.sleep(0.3)

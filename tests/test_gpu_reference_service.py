@@ -1,4 +1,4 @@
-"""The UNMODIFIED reference service (baseline/_ref, or /root/reference/src in the build container) around the real
+"""The UNMODIFIED reference service (oracle/_ref, see oracle/Makefile) around the real
 CUDA library.  Needs a B200.  Covers SURVEY.md 8(a3), 8(b): both plugin routes -- the component loader
 (settings.component_type = dotted path; /root/reference/src/service/features/component_loader.py:34-55) and the
 Service subclass (core.py:64-69,85-86) -- with the reference's own metrics (core.py:184-200) asserted."""
@@ -13,20 +13,12 @@ import pytest
 from detectmateservice_b200 import wire
 from detectmateservice_b200.compat import install_shims
 from oracle.native import NativeOracle
+from oracle.ref_engine import reference_path as _reference_src
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-
-def _reference_src():
-    for p in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference/src"):
-        if os.path.isdir(os.path.join(p, "service")):
-            return p
-    return None
-
-
-needs_ref = pytest.mark.skipif(_reference_src() is None, reason="the reference service is not installed (baseline/_ref)")
+needs_ref = pytest.mark.skipif(_reference_src() is None, reason="the reference service is not in oracle/_ref (make -C oracle ref)")
 
 
 def _metric(counter, **labels):
@@ -34,7 +26,7 @@ def _metric(counter, **labels):
 
 
 @needs_ref
-def test_reference_service_loads_the_cuda_component(tmp_path, monkeypatch, golden_dir):
+def test_reference_service_loads_the_cuda_component(tmp_path, sock_dir, monkeypatch, golden_dir):
     import yaml
     monkeypatch.syspath_prepend(_reference_src())
     install_shims()
@@ -47,7 +39,7 @@ def test_reference_service_loads_the_cuda_component(tmp_path, monkeypatch, golde
     cfg_file = tmp_path / "detector_config.yaml"
     det_cfg = dict(g["config"]["detectors"]["NewValueDetector"])
     cfg_file.write_text(yaml.safe_dump({"detectors": {"B200NewValueDetector": det_cfg}}))
-    addr = f"ipc://{tmp_path}/svc.ipc"
+    addr = f"ipc://{sock_dir}/svc.ipc"
     settings = ServiceSettings(component_type="detectmateservice_b200.component.B200NewValueDetector",
                                component_name="b200-det-gpu", engine_addr=addr, config_file=cfg_file,
                                log_dir=tmp_path / "logs", log_to_file=False, log_to_console=False,
@@ -84,7 +76,7 @@ def test_reference_service_loads_the_cuda_component(tmp_path, monkeypatch, golde
 
 
 @needs_ref
-def test_service_subclass_route_on_raw_batches(tmp_path, monkeypatch):
+def test_service_subclass_route_on_raw_batches(tmp_path, sock_dir, monkeypatch):
     """b200_detector_service(): a Service subclass whose process() keeps the base class's metrics; fed with raw
     key=value batches (one message = many records), checked against the oracle."""
     monkeypatch.syspath_prepend(_reference_src())
@@ -106,7 +98,7 @@ def test_service_subclass_route_on_raw_batches(tmp_path, monkeypatch):
         "params": {"output_format": "compact", "max_batch_bytes": 4 << 20},
         "global": {"g": {"header_variables": [{"pos": k} for k in MONITORED_KEYS]}}}}}
     Svc = b200_detector_service()
-    settings = ServiceSettings(component_name="b200-subclass", engine_addr=f"ipc://{tmp_path}/sub.ipc",
+    settings = ServiceSettings(component_name="b200-subclass", engine_addr=f"ipc://{sock_dir}/sub.ipc",
                                log_dir=tmp_path / "logs", log_to_file=False, log_to_console=False,
                                http_port=18232, engine_autostart=False)
     svc = Svc(settings=settings, component_config=cfg)

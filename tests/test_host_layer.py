@@ -26,8 +26,7 @@ import pynng  # noqa: E402
 from oracle import schemas as oschemas  # noqa: E402
 from oracle.native import NativeOracle  # noqa: E402
 
-REF_SRC = next((p for p in (os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref"),
-                             "/root/reference/src") if os.path.isdir(os.path.join(p, "service"))), "/root/reference/src")
+from oracle.ref_engine import REF_DIR as REF_SRC  # noqa: E402
 
 
 # ------------------------------------------------------------------------------------------
@@ -63,12 +62,12 @@ def test_wire_detector_schema_roundtrip_with_protobuf():
 # ------------------------------------------------------------------------------------------
 # SP / PAIR0 transport
 # ------------------------------------------------------------------------------------------
-def test_pair0_wire_format_tcp_and_ipc(tmp_path):
+def test_pair0_wire_format_tcp_and_ipc(sock_dir):
     """The bytes on the wire are NNG's: 8-byte SP header, PAIR0 = 0x0010, be64 length frames
     (ipc frames carry a leading 0x01)."""
     if not getattr(pynng, "__shim__", False):
         pytest.skip("real pynng installed")
-    for addr in ("tcp://127.0.0.1:0", f"ipc://{tmp_path}/w.ipc"):
+    for addr in ("tcp://127.0.0.1:0", f"ipc://{sock_dir}/w.ipc"):
         srv = pynng.Pair0(recv_timeout=2000)
         if addr.startswith("tcp"):
             s0 = socket.socket()
@@ -98,8 +97,8 @@ def test_pair0_wire_format_tcp_and_ipc(tmp_path):
         srv.close()
 
 
-def test_pair0_semantics(tmp_path):
-    addr = f"ipc://{tmp_path}/p.ipc"
+def test_pair0_semantics(sock_dir):
+    addr = f"ipc://{sock_dir}/p.ipc"
     with pynng.Pair0(recv_timeout=100) as a:
         with pytest.raises(pynng.TryAgain):
             a.send(b"x", block=False)                      # no peer
@@ -122,8 +121,8 @@ def test_pair0_semantics(tmp_path):
         a.send(b"closed")
 
 
-def test_pair0_late_binding_and_reconnect(tmp_path):
-    addr = f"ipc://{tmp_path}/late.ipc"
+def test_pair0_late_binding_and_reconnect(sock_dir):
+    addr = f"ipc://{sock_dir}/late.ipc"
     out = pynng.Pair0()
     out.dial(addr, block=False)                            # nobody listens yet
     with pytest.raises(pynng.TryAgain):
@@ -140,11 +139,11 @@ def test_pair0_late_binding_and_reconnect(tmp_path):
     out.close()
 
 
-def test_pair0_nonblocking_send_queues_and_oversize_frames(tmp_path):
+def test_pair0_nonblocking_send_queues_and_oversize_frames(sock_dir):
     """send(block=False) to a connected peer that is not draining does not drop (the reference's
     fan-out, engine.py:234-243, relies on it: tests/test_service_multi_output_integration.py:298-318);
     unknown transports are NotSupported; recv_max_size closes the connection on an oversized frame."""
-    addr = f"ipc://{tmp_path}/q.ipc"
+    addr = f"ipc://{sock_dir}/q.ipc"
     with pynng.Pair0(listen=addr, recv_timeout=2000) as rx, pynng.Pair0(recv_timeout=2000) as tx:
         tx.send_buffer_size = 0
         tx.dial(addr, block=True)
@@ -159,7 +158,7 @@ def test_pair0_nonblocking_send_queues_and_oversize_frames(tmp_path):
         assert rx.recv() == big and rx.recv() == b"after"
     with pytest.raises(pynng.exceptions.NotSupported):
         pynng.Pair0(listen="invalid://address")
-    addr2 = f"ipc://{tmp_path}/m.ipc"
+    addr2 = f"ipc://{sock_dir}/m.ipc"
     with pynng.Pair0(listen=addr2, recv_timeout=300) as rx, pynng.Pair0(dial=addr2) as tx:
         rx.recv_max_size = 1024
         time.sleep(0.05)
@@ -190,9 +189,9 @@ class _Upper:
         return None if raw == b"skip" else raw.upper()
 
 
-def test_engine_mirror_reply_none_exception_and_fanout(tmp_path):
+def test_engine_mirror_reply_none_exception_and_fanout(sock_dir):
     from detectmateservice_b200.service import DetectorEngine
-    eng_addr = f"ipc://{tmp_path}/e.ipc"
+    eng_addr = f"ipc://{sock_dir}/e.ipc"
     with DetectorEngine(_Upper(), eng_addr) as eng:
         with pynng.Pair0(dial=eng_addr, recv_timeout=1000) as c:
             c.send(b"hi")
@@ -208,9 +207,9 @@ def test_engine_mirror_reply_none_exception_and_fanout(tmp_path):
             c.send(b"again")
             assert c.recv() == b"AGAIN"
         assert eng.counters["errors"] == 1 and eng.counters["messages"] == 4
-    outs = [f"ipc://{tmp_path}/o{i}.ipc" for i in range(3)]
+    outs = [f"ipc://{sock_dir}/o{i}.ipc" for i in range(3)]
     sinks = [pynng.Pair0(listen=o, recv_timeout=2000) for o in outs[:2]]      # third output never comes up
-    eng2_addr = f"ipc://{tmp_path}/e2.ipc"
+    eng2_addr = f"ipc://{sock_dir}/e2.ipc"
     with DetectorEngine(_Upper(), eng2_addr, out_addr=outs) as eng:
         time.sleep(0.3)
         with pynng.Pair0(dial=eng2_addr) as c:
@@ -448,8 +447,8 @@ def test_component_reconfigure_decides_what_has_to_be_rebuilt():
     assert c.logformat is not None                               # a rejected configuration changes nothing
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="the reference service is neither in baseline/_ref nor in /root/reference/src")
-def test_service_subclass_forwards_reconfigure(tmp_path, monkeypatch):
+@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="the reference service is not in oracle/_ref (make -C oracle ref)")
+def test_service_subclass_forwards_reconfigure(tmp_path, sock_dir, monkeypatch):
     """Service.reconfigure (core.py:299-345) stores the new configuration; the B200 subclass hands it to the
     detector before the next message (the device handle is a double here)."""
     import yaml
@@ -462,7 +461,7 @@ def test_service_subclass_forwards_reconfigure(tmp_path, monkeypatch):
     cfg_file = tmp_path / "detector_config.yaml"
     cfg_file.write_text(yaml.safe_dump(det_cfg(["type"], 1)))
     Svc = b200_detector_service()
-    svc = Svc(settings=ServiceSettings(component_name="b200-reconf", engine_addr=f"ipc://{tmp_path}/r.ipc", config_file=cfg_file,
+    svc = Svc(settings=ServiceSettings(component_name="b200-reconf", engine_addr=f"ipc://{sock_dir}/r.ipc", config_file=cfg_file,
                                        log_dir=tmp_path / "logs", log_to_file=False, log_to_console=False, http_port=18127,
                                        engine_autostart=False))
     try:
@@ -493,8 +492,8 @@ def test_service_subclass_forwards_reconfigure(tmp_path, monkeypatch):
 # ------------------------------------------------------------------------------------------
 # the UNMODIFIED reference service, with the shims, loading the B200 component
 # ------------------------------------------------------------------------------------------
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="the reference service is neither in baseline/_ref nor in /root/reference/src")
-def test_reference_service_loads_b200_component(tmp_path, monkeypatch, golden_dir):
+@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="the reference service is not in oracle/_ref (make -C oracle ref)")
+def test_reference_service_loads_b200_component(tmp_path, sock_dir, monkeypatch, golden_dir):
     import yaml
     monkeypatch.syspath_prepend(REF_SRC)
     from service.core import Service                     # reference code, imported unmodified
@@ -514,7 +513,7 @@ def test_reference_service_loads_b200_component(tmp_path, monkeypatch, golden_di
         self._det = FakeDevice([m.key for m in self.monitors])
     monkeypatch.setattr(comp_mod.B200NewValueDetector, "__init__", init)
 
-    addr = f"ipc://{tmp_path}/svc.ipc"
+    addr = f"ipc://{sock_dir}/svc.ipc"
     settings = ServiceSettings(component_type="detectmateservice_b200.component.B200NewValueDetector",
                                component_name="b200-det", engine_addr=addr, config_file=cfg_file,
                                log_dir=tmp_path / "logs", log_to_file=False, log_to_console=False,
@@ -593,7 +592,7 @@ class _ParserStage:
                                           "logFormatVariables": fields})
 
 
-def test_config1_reader_parser_detector_pipeline(tmp_path, golden_dir):
+def test_config1_reader_parser_detector_pipeline(sock_dir, golden_dir):
     from detectmateservice_b200.service import DetectorEngine
     exp = json.load(open(os.path.join(golden_dir, "audit_sample.expected.json")))
     lines = open(os.path.join(golden_dir, "audit_sample.log"), "rb").read().split(b"\n")[:-1]
@@ -601,7 +600,7 @@ def test_config1_reader_parser_detector_pipeline(tmp_path, golden_dir):
         "method_type": "new_value_detector", "data_use_training": exp["n_train"], "auto_config": False,
         "global": {"g": {"header_variables": [{"pos": k} for k in exp["keys"]]}}}}}
     det = _component(cfg)
-    a_reader, a_parser, a_det, a_out = (f"ipc://{tmp_path}/{n}.ipc" for n in ("reader", "parser", "detector", "out"))
+    a_reader, a_parser, a_det, a_out = (f"ipc://{sock_dir}/{n}.ipc" for n in ("reader", "parser", "detector", "out"))
     sink = pynng.Pair0(listen=a_out, recv_timeout=300)
     with DetectorEngine(det, a_det, out_addr=[a_out]) as e_det, \
             DetectorEngine(_ParserStage(), a_parser, out_addr=[a_det]), \
@@ -631,7 +630,7 @@ def test_config1_reader_parser_detector_pipeline(tmp_path, golden_dir):
         assert a["extractedTimestamps"][0] > 1600000000
 
 
-def test_engine_lends_receive_frames(tmp_path, golden_dir):
+def test_engine_lends_receive_frames(sock_dir, golden_dir):
     """alloc_frame / release_frame: the engine hands the transport the processor's receive
     buffers for large messages and gives each one back after process() (also on errors)."""
     from detectmateservice_b200.service import DetectorEngine
@@ -668,7 +667,7 @@ def test_engine_lends_receive_frames(tmp_path, golden_dir):
             return None
 
     p = Lender()
-    addr = f"ipc://{tmp_path}/lend.ipc"
+    addr = f"ipc://{sock_dir}/lend.ipc"
     msgs = [bytes([65 + i]) * (200000 + i) for i in range(6)] + [b"boom" * 50000, b"small", b"Z" * (2 << 20)]
     with DetectorEngine(p, addr) as e, pynng.Pair0(dial=addr) as s:
         time.sleep(0.2)

@@ -1,13 +1,8 @@
 """Wire schema pins: the 201-byte ParserSchema fixture and the reference descriptor."""
 import json
 import os
-import re
-
-import pytest
 
 from oracle.schemas import ParserSchema, build_file_descriptor, parser_schema_from_dict
-
-REF_RB = "/root/reference/container/fluentout/schemas_pb.rb"
 
 
 def test_parser_fixture1_wire_image(golden_dir):
@@ -22,40 +17,15 @@ def test_parser_fixture1_wire_image(golden_dir):
     assert m.receivedTimestamp == 1634567890 and m.parsedTimestamp == 1634567891
 
 
-def _ruby_unescape(s: str) -> bytes:
-    out = bytearray()
-    i = 0
-    simple = {"n": 10, "r": 13, "t": 9, '"': 34, "\\": 92, "e": 27, "a": 7, "b": 8, "f": 12, "v": 11, "0": 0, "#": 35}
-    while i < len(s):
-        c = s[i]
-        if c != "\\":
-            out += c.encode("latin-1")
-            i += 1
-            continue
-        n = s[i + 1]
-        if n == "x":
-            m = re.match(r"[0-9a-fA-F]{1,2}", s[i + 2:i + 4])
-            out.append(int(m.group(0), 16))
-            i += 2 + len(m.group(0))
-        elif n in "01234567":
-            m = re.match(r"[0-7]{1,3}", s[i + 1:i + 4])
-            out.append(int(m.group(0), 8))
-            i += 1 + len(m.group(0))
-        else:
-            out.append(simple[n])
-            i += 2
-    return bytes(out)
-
-
-@pytest.mark.skipif(not os.path.exists(REF_RB), reason="reference checkout not present (GPU box)")
-def test_restated_schema_equals_reference_descriptor():
+def test_restated_schema_equals_reference_descriptor(golden_dir):
     """Field names, numbers, types and labels of LogSchema/ParserSchema/DetectorSchema equal
-    the descriptor embedded in container/fluentout/schemas_pb.rb:8."""
+    the descriptor embedded in the reference's container/fluentout/schemas_pb.rb:8 (stored in
+    schemas_descriptor.json by scripts/make_golden.py)."""
     from google.protobuf import descriptor_pb2
-    src = open(REF_RB, "r", encoding="latin-1").read()
-    lit = re.search(r'descriptor_data = "((?:[^"\\]|\\.)*)"', src, re.S).group(1)
+    g = json.load(open(os.path.join(golden_dir, "schemas_descriptor.json")))
     ref = descriptor_pb2.FileDescriptorProto()
-    ref.ParseFromString(_ruby_unescape(lit))
+    ref.ParseFromString(bytes.fromhex(g["file_descriptor_hex"]))
+    assert {"LogSchema", "ParserSchema", "DetectorSchema"} <= {m.name for m in ref.message_type}
     mine = build_file_descriptor()
     ref_msgs = {m.name: m for m in ref.message_type}
     for m in mine.message_type:
